@@ -8,7 +8,8 @@ reference-facing C-ABI call ``hived_process_events`` with pinned HOST buffers (H
 of the results inside the timed region).  ``--impl reference`` times the reference's own CPU algorithm
 (the oracle: a faithful C++ restatement of the Go path; Go itself is not available in this image).
 
-One JSON line is printed by rank 0.
+One JSON line is printed by rank 0.  ``--dump-outputs DIR`` also writes the results of the last timed step as .npy
+files, so that two builds can be compared output for output on the same seeded trace.
 """
 import argparse
 import ctypes as C
@@ -23,6 +24,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: the benchmark writes nothing into it
 
 from hivedscheduler_b200 import _cabi, trace  # noqa: E402
 
@@ -89,6 +91,33 @@ def bind_bench_hooks(lib):
         fn = getattr(lib, name)
         fn.restype = res
         fn.argtypes = args
+
+
+DUMP_BUDGET_BYTES = 60_000_000  # array data of --dump-outputs; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, res, pool):
+    """What hived_process_events hands its caller for the batch: one float64 file per field of hived_result_t
+    (result_<field>.npy, one row per event; int32 values are exact in float64) and the result pool (pool.npy).
+    result_index.npy / pool_index.npy name the event rows and pool words written: all of them when they fit
+    DUMP_BUDGET_BYTES, otherwise the same fixed seeded sample of both, sorted, for every run of the same trace."""
+    os.makedirs(out_dir, exist_ok=True)
+    cols = sum(int(np.prod(res.dtype[f].shape)) for f in res.dtype.names)
+    rows, words = len(res), len(pool)
+    values = rows * (cols + 1) + words * 2  # +1 / *2: the index arrays
+    cap = DUMP_BUDGET_BYTES // 8
+    rng = np.random.default_rng(0)
+
+    def pick(n):
+        k = n if values <= cap else int(n * cap / values)
+        return np.arange(n) if k == n else np.sort(rng.choice(n, k, replace=False))
+
+    ri, pi = pick(rows), pick(words)
+    np.save(os.path.join(out_dir, "result_index.npy"), ri.astype(np.float64))
+    for f in res.dtype.names:
+        np.save(os.path.join(out_dir, "result_%s.npy" % f), res[f][ri].astype(np.float64))
+    np.save(os.path.join(out_dir, "pool_index.npy"), pi.astype(np.float64))
+    np.save(os.path.join(out_dir, "pool.npy"), pool[pi].astype(np.float64))
 
 
 def dist_env():
@@ -481,7 +510,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--replicas", action="store_true", help="N > 1: independent replicas (weak scaling) instead of the VC partition")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the C2 / C4 / C5 sub-lines (about 45 s)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step to DIR/<name>.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl == "reference" or (dist_env()[1] > 1 and not args.replicas)):
+        ap.error("--dump-outputs writes the results of one whole batch: --impl ours on one GPU or with --replicas")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -558,7 +593,11 @@ def main():
     n_ctas = lib.hived_bench_num_ctas(ctx)
     # parity witness: the hash of the last step's results
     used = C.c_int64()
-    lib.hived_bench_fetch_results(ctx, res_ptr, pool_ptr, pool_words, C.byref(used))
+    rc = lib.hived_bench_fetch_results(ctx, res_ptr, pool_ptr, pool_words, C.byref(used))
+    assert rc == 0, rc
+    if args.dump_outputs:  # copies: the legs below reuse the pinned buffers
+        last_res = np.frombuffer(res_pinned.numpy(), dtype=trace.RESULT_DT).copy()
+        last_pool = pool_pinned.numpy()[:used.value].copy()
     stats = bc.stats()
     cyc = (C.c_int64 * 15)()
     lib.hived_bench_phase_cycles(ctx, cyc)
@@ -659,6 +698,8 @@ def main():
             line["phase_cycles_per_step"] = {n: int(c) for n, c in zip(names, cyc)}
         if os.environ.get("HIVED_BENCH_DEBUG"):
             line["debug_cycles"] = [int(x) for x in dbg]
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_res, last_pool)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -1,5 +1,6 @@
-import sys, time, json
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tests')
+import os, sys, time, json
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 from hivedscheduler_b200 import trace, _cabi
 lib = _cabi.load_cuda_library()
 out = {}
@@ -20,7 +21,7 @@ out["C2"] = {"decisions": len(t["events"]), "seconds_e2e": dt, "decisions_per_s"
 bc.close()
 # C4: call-by-call harness (includes the Python harness itself)
 from importlib import util
-spec = util.spec_from_file_location("g", "/root/repo/tests/golden/make_trace_hashes.py"); g = util.module_from_spec(spec); spec.loader.exec_module(g)
+spec = util.spec_from_file_location("g", os.path.join(ROOT, "tests", "golden", "make_trace_hashes.py")); g = util.module_from_spec(spec); spec.loader.exec_module(g)
 t0 = time.perf_counter(); h, log, st = trace.run_c4_interactive(lib, **g.c4_kwargs(100000)); dt = time.perf_counter() - t0
 out["C4"] = {"gangs": 100000, "calls": st["schedule_events"], "seconds_wall_incl_python_harness": dt, "gangs_per_s": 100000 / dt, "hash": "%016x" % h}
 print(json.dumps(out, indent=1))

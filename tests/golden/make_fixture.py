@@ -1,16 +1,16 @@
 #!/usr/bin/env python
 """Generates tests/golden/hived_algorithm_test.json from the reference's own test file and fixture.
 
-Run in the build container only (it reads /root/reference, which does not exist on the GPU box):
+Needs a checkout of microsoft/hivedscheduler; the tests only read the committed JSON:
 
-    python tests/golden/make_fixture.py
+    python tests/golden/make_fixture.py <hivedscheduler checkout>
 
 Extracted verbatim (data only, no code) from
-  /root/reference/pkg/algorithm/hived_algorithm_test.go
+  pkg/algorithm/hived_algorithm_test.go
     group1..group34 (:66-170), pss (:172-542), casesThatShouldSucceed/Fail/BeLazyPreempted,
     casesForStatefulPreemption (:544-560), expectedBindInfos (:566-592), expectedPreemptInfos (:594-602),
     deletedPreemptorGroups (:604-608)
-  /root/reference/example/config/design/hivedscheduler.yaml (the cluster the vectors are defined on)
+  example/config/design/hivedscheduler.yaml (the cluster the vectors are defined on)
 The scenario (call order, config edits, assertions) is restated in tests/golden_scenario.py.
 """
 import json
@@ -20,14 +20,11 @@ import sys
 
 import yaml
 
-REF = "/root/reference"
-TEST_GO = os.path.join(REF, "pkg/algorithm/hived_algorithm_test.go")
-DESIGN_YAML = os.path.join(REF, "example/config/design/hivedscheduler.yaml")
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "hived_algorithm_test.json")
 
 
-def main():
-    src = open(TEST_GO).read()
+def main(ref):
+    src = open(os.path.join(ref, "pkg/algorithm/hived_algorithm_test.go")).read()
     # ---- affinity group specs
     groups = {}
     for m in re.finditer(r'Name:\s+"(group\d+)",\s*Members:\s*\[\]api\.AffinityGroupMemberSpec\{(.*?)\},\n', src):
@@ -85,7 +82,7 @@ def main():
     del_src = re.search(r"var deletedPreemptorGroups = map\[string\]\[\]string\{(.*?)\n\}", src, re.S).group(1)
     deleted = {mm.group(1): re.findall(r'"([^"]+)"', mm.group(2))
                for mm in re.finditer(r'"(pod\d+)": \{([^}]*)\}', del_src)}
-    design = yaml.safe_load(open(DESIGN_YAML))
+    design = yaml.safe_load(open(os.path.join(ref, "example/config/design/hivedscheduler.yaml")))
     out = {
         "source": "microsoft/hivedscheduler pkg/algorithm/hived_algorithm_test.go + example/config/design/hivedscheduler.yaml",
         "design_config": {"physicalCluster": design["physicalCluster"], "virtualClusters": design["virtualClusters"]},
@@ -104,4 +101,6 @@ def main():
 
 
 if __name__ == "__main__":
-    sys.exit(main())
+    if len(sys.argv) != 2:
+        sys.exit("usage: make_fixture.py <hivedscheduler checkout>")
+    sys.exit(main(sys.argv[1]))

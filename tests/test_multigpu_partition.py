@@ -177,7 +177,8 @@ def test_bench_partitioned_leg_plumbing_over_gloo(emu_mt_lib, oracle_lib):
     s.bind(("127.0.0.1", 0))
     port = s.getsockname()[1]
     s.close()
-    env = dict(os.environ, HIVED_BENCH_PLUMBING_TEST_LIB=emu_mt_lib._name)
+    # bench.py takes the emulation path only without a visible GPU: hide any, so both ranks run it on every machine
+    env = dict(os.environ, HIVED_BENCH_PLUMBING_TEST_LIB=emu_mt_lib._name, CUDA_VISIBLE_DEVICES="")
     out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
                           "--master-port", str(port), os.path.join(ROOT, "bench.py"), "--gpus", "2", "--steps", "1", "--warmup", "1",
                           "--gangs", "1200"], env=env, capture_output=True, text=True, timeout=600)
