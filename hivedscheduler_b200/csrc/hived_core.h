@@ -423,9 +423,13 @@ struct Core {
   }
   HIVED_DEV bool fl_contains(int cell) const { return d.p_flpos[cell] >= 0; }
   // ---- bad free cells (badFreeCells, hived_algorithm.go:78)
+  // Its segment has the free list's capacity (fl_cap).  A cell can be listed only once here (p_bfpos is its position):
+  // a second append — the reference's slice would take it — and an append to a full segment report HIVED_ERR_CAPACITY
+  // instead of writing into the neighbouring segment.
   HIVED_DEV void bf_append(int chain, int level, int cell) {
     int k = cl(chain, level);
     int n = d.bf_len[k];
+    if (n >= d.fl_cap[k] || d.p_bfpos[cell] >= 0) { panic(HIVED_ERR_CAPACITY); return; }
     hv_warp_sync();
     ST(d.bf_data[d.fl_base[k] + n], cell);
     ST(d.p_bfpos[cell], n);
@@ -444,10 +448,15 @@ struct Core {
     ST(d.bf_len[k], n - 1);
   }
   // ---- doomed bad cells of a VC (vcDoomedBadCells, hived_algorithm.go:80)
+  // The reference's list keeps STALE entries: a doomed bad cell that a pod used is unbound when the pod leaves
+  // (releaseLeafCell unbinds it but skips releasePreassignedCell because the cell is still listed), its virtual cell can
+  // be bound to another bad cell, and the list outgrows the VC's preassigned cells (synthetic fuzz seed 2098).  The
+  // segment has room for DM_STALE_SLACK such entries (hived_topo.hpp); beyond that, or for a cell that is already on a
+  // doomed bad list (p_dmpos / p_dmvc hold one position per cell), the call reports HIVED_ERR_CAPACITY.
   HIVED_DEV void dm_append(int vc, int chain, int level, int cell) {
     int k = vcl(vc, chain, level);
     int n = d.dm_len[k];
-    if (n >= d.dm_cap[k]) { panic(HIVED_ERR_PLATFORM); return; }
+    if (n >= d.dm_cap[k] || d.p_dmpos[cell] >= 0) { panic(HIVED_ERR_CAPACITY); return; }
     hv_warp_sync();
     ST(d.dm_data[d.dm_base[k] + n], cell);
     ST(d.p_dmpos[cell], n);
@@ -697,7 +706,9 @@ struct Core {
       int kv = vcl(vc, chain, l);
       int guard = 0;
       while (d.vcFree[kv] > d.totalLeft[k] - d.bf_len[k]) {
-        if (d.bf_len[k] <= 0 || ++guard > d.S.NP) { panic(HIVED_ERR_PLATFORM); return; }
+        if (d.bf_len[k] <= 0) { panic(HIVED_ERR_PLATFORM); return; }  // badFreeCells[c][l][0] of an empty slice in the reference
+        // a device limit, not the reference's: it would go on binding (one bad free cell per round, each leaves the list)
+        if (++guard > d.S.NP) { panic(HIVED_ERR_CAPACITY); return; }
         int pc = d.bf_data[d.fl_base[k] + 0];
         const int32_t* pre = d.pre_list + d.pre_off[kv];
         int idx = firstIdx(d.pre_cnt[kv], [&](int i) { return d.v_pcell[pre[i]] < 0; });
@@ -722,7 +733,7 @@ struct Core {
       int kv = vcl(vc, chain, l);
       int guard = 0;
       while (d.dm_len[kv] != 0 && d.vcFree[kv] < d.totalLeft[k] - d.bf_len[k]) {
-        if (++guard > d.S.NP) { panic(HIVED_ERR_PLATFORM); return; }
+        if (++guard > d.S.NP) { panic(HIVED_ERR_CAPACITY); return; }  // a device limit: every round takes one entry off the list
         int pc = d.dm_data[d.dm_base[kv] + 0];
         if (d.p_vcell[pc] < 0) { panic(HIVED_ERR_PLATFORM); return; }  // nil virtual cell dereferenced in the reference (:643-646)
         unbindPair(pc, d.p_vcell[pc]);
@@ -1454,7 +1465,8 @@ struct Core {
     const int HIGHEST = 0x7fffffff;
     int bestAffinity = HIGHEST;
     int optimal = optimalAffinity(chain, k);
-    if (optimal < 0 || k > MAX_NODE_LEAVES) { panic(HIVED_ERR_PLATFORM); return; }
+    if (k > MAX_NODE_LEAVES) { panic(HIVED_ERR_CAPACITY); return; }  // the search's arrays (a device limit)
+    if (optimal < 0) { panic(HIVED_ERR_PLATFORM); return; }
     int ai = 0, si = 0;
     bool done = false;
     while (!done) {

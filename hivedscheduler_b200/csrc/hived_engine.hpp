@@ -9,11 +9,13 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 #include <memory>
 #include <string>
 #include <vector>
 
 #include "../../include/hived.h"
+#include "../../include/hived_bench.h"
 #include "../../include/hived_hash.h"
 #include "../../include/hived_multigpu.h"
 #include "hived_topo.hpp"
@@ -769,13 +771,19 @@ int hived_get_group(hived_ctx* ctx, int32_t group, hived_group_info_t* out) {
   hived::bk_d2h(hdr, e.dev.g_hdr + (size_t)group * hived::GROUP_HDR_WORDS, sizeof hdr);
   int32_t v[5] = {hdr[0], hdr[1], hdr[2], hdr[3], hdr[5]};
   if (v[0] == HIVED_GROUP_NONE) {
-    // an erased object of this id that cells may still name (Core::ghostify): the shims keep the id (hived.h "Id lifetime")
-    const int32_t slot = hdr[hived::GH_LINK] - 1;
-    if (slot >= e.dev.S.maxGroups && slot < e.dev.S.maxGroups + hived::GHOST_GROUPS) {
-      int32_t gh[hived::GROUP_HDR_WORDS];
-      hived::bk_d2h(gh, e.dev.g_hdr + (size_t)slot * hived::GROUP_HDR_WORDS, sizeof gh);
-      if (gh[0] != HIVED_GROUP_NONE && gh[hived::GH_ORIGIN] == group + 1) out->referenced = 1;
-    }
+    // an erased object of this id that cells may still name (Core::ghostify): the shims keep the id (hived.h "Id lifetime").
+    // Every cell is looked at, like the reference's pointers would be: a ghost that was itself erased by name
+    // (Core::eraseGroupByName) has state NONE but its cells still name it, and a later erase through them hits this id.
+    const int32_t G = e.dev.S.maxGroups;
+    std::vector<int32_t> usingG, resv, gh;
+    e.readArray(e.dev.p_using, usingG, e.T.NP); e.readArray(e.dev.p_resv, resv, e.T.NP);
+    e.readArray(e.dev.g_hdr + (size_t)G * hived::GROUP_HDR_WORDS, gh, (size_t)hived::GHOST_GROUPS * hived::GROUP_HDR_WORDS);
+    auto names = [&](int32_t s) {
+      if (s == group) return true;
+      return s >= G && s < G + hived::GHOST_GROUPS && gh[(size_t)(s - G) * hived::GROUP_HDR_WORDS + hived::GH_ORIGIN] == group + 1;
+    };
+    for (int c = 0; c < e.T.NP && !out->referenced; c++)
+      if (names(usingG[c]) || names(resv[c])) out->referenced = 1;
     return 0;
   }
   out->state = v[0]; out->vc = v[1]; out->priority = v[2];
@@ -1009,6 +1017,107 @@ uint64_t hived_debug_view_hash(hived_ctx* ctx) {
     total += h;
   }
   return total;
+}
+/* test hook: the scheduler state that decides LATER calls and that neither a result nor a cell snapshot shows, in the
+   canonical encoding of include/hived_bench.h (tagged sections, zeros and missing map entries omitted).  Derived the
+   way the device program reads it: the used-leaf counters from the leaf priorities plus the recorded drift
+   (noteDelta), the opportunistic count of a physical cell from p_usedopp, a ghost group record as its origin id. */
+int64_t hived_debug_state(hived_ctx* ctx, int32_t* out, int64_t cap) {
+  hived::Engine& e = ctx->e;
+  const hived::FlatTopo& T = e.T;
+  const auto& S = e.dev.S;
+  using hived::MAXL;
+  const size_t CL = (size_t)S.nChains * MAXL, VCL = (size_t)S.nVCs * CL;
+  std::vector<int32_t> fl, fll, bf, bfl, dm, dml, vcf, allf, tl, ad;
+  e.readArray(e.dev.fl_data, fl, S.flTotal); e.readArray(e.dev.fl_len, fll, CL);
+  e.readArray(e.dev.bf_data, bf, S.flTotal); e.readArray(e.dev.bf_len, bfl, CL);
+  e.readArray(e.dev.dm_data, dm, S.dmTotal); e.readArray(e.dev.dm_len, dml, VCL);
+  e.readArray(e.dev.vcFree, vcf, VCL); e.readArray(e.dev.allVCFree, allf, CL);
+  e.readArray(e.dev.totalLeft, tl, CL); e.readArray(e.dev.allVCDoomed, ad, CL);
+  std::vector<int32_t> o;
+  auto list = [&](std::initializer_list<int32_t> head, const std::vector<int32_t>& data, int32_t base, int32_t n) {
+    if (n == 0) return;
+    o.insert(o.end(), head); o.push_back(n);
+    for (int32_t i = 0; i < n; i++) o.push_back(data[(size_t)base + i]);
+  };
+  for (int c = 0; c < S.nChains; c++)
+    for (int l = 1; l < MAXL; l++) list({HIVED_DS_FREE, c, l}, fl, T.fl_base[c * MAXL + l], fll[c * MAXL + l]);
+  for (int c = 0; c < S.nChains; c++)
+    for (int l = 1; l < MAXL; l++) list({HIVED_DS_BAD_FREE, c, l}, bf, T.fl_base[c * MAXL + l], bfl[c * MAXL + l]);
+  for (int v = 0; v < S.nVCs; v++)
+    for (int c = 0; c < S.nChains; c++)
+      for (int l = 1; l < MAXL; l++) {
+        const size_t k = ((size_t)v * S.nChains + c) * MAXL + l;
+        list({HIVED_DS_DOOMED_BAD, v, c, l}, dm, T.dm_base[k], dml[k]);
+      }
+  for (int v = 0; v < S.nVCs; v++)
+    for (int c = 0; c < S.nChains; c++) {
+      if (!T.vc_chain_counter[(size_t)v * S.nChains + c]) continue;
+      for (int l = 1; l < MAXL; l++) {
+        const int32_t x = vcf[((size_t)v * S.nChains + c) * MAXL + l];
+        if (x) o.insert(o.end(), {HIVED_DS_VC_FREE, v, c, l, x});
+      }
+    }
+  const std::pair<int32_t, const std::vector<int32_t>*> perChain[] = {
+      {HIVED_DS_ALL_VC_FREE, &allf}, {HIVED_DS_TOTAL_LEFT, &tl}, {HIVED_DS_ALL_VC_DOOMED, &ad}};
+  for (const auto& t : perChain)
+    for (int c = 0; c < S.nChains; c++)
+      for (int l = 1; l < MAXL; l++) {
+        const int32_t x = (*t.second)[c * MAXL + l];
+        if (x) o.insert(o.end(), {t.first, c, l, x});
+      }
+  // used-leaf counters: (priority, count) per cell, ascending priority
+  auto used = [&](bool virt, int n, int32_t tag) {
+    std::vector<int32_t> prio, dprio, dcnt, opp;
+    e.readArray(virt ? e.dev.v_prio : e.dev.p_prio, prio, n);
+    e.readArray(virt ? e.dev.v_dprio : e.dev.p_dprio, dprio, (size_t)n * hived::DELTA_SLOTS);
+    e.readArray(virt ? e.dev.v_dcnt : e.dev.p_dcnt, dcnt, (size_t)n * hived::DELTA_SLOTS);
+    if (!virt) e.readArray(e.dev.p_usedopp, opp, n);
+    const std::vector<int32_t>& level = virt ? T.v_level : T.p_level;
+    const std::vector<int32_t>& parent = virt ? T.v_parent : T.p_parent;
+    std::vector<std::map<int32_t, int32_t>> m(n);
+    for (int c = 0; c < n; c++) {
+      if (level[c] != 1 || prio[c] == hived::FREE_PRIO) continue;
+      if (!virt && prio[c] == hived::OPP_PRIO) continue;  // counted by p_usedopp
+      for (int a = c; a >= 0; a = parent[a]) m[a][prio[c]]++;
+    }
+    for (int c = 0; c < n; c++) {
+      for (int i = 0; i < hived::DELTA_SLOTS; i++) {
+        const int32_t p = dprio[(size_t)c * hived::DELTA_SLOTS + i];
+        if (p == hived::DELTA_EMPTY || (!virt && p == hived::OPP_PRIO)) continue;
+        m[c][p] += dcnt[(size_t)c * hived::DELTA_SLOTS + i];
+      }
+      if (!virt) m[c][hived::OPP_PRIO] += opp[c];
+      int32_t k = 0;
+      for (const auto& kv : m[c]) k += kv.second != 0;
+      if (k == 0) continue;
+      o.insert(o.end(), {tag, c, k});
+      for (const auto& kv : m[c]) if (kv.second != 0) o.insert(o.end(), {kv.first, kv.second});
+    }
+  };
+  used(false, T.NP, HIVED_DS_USED_PHYSICAL);
+  used(true, T.NV, HIVED_DS_USED_VIRTUAL);
+  // using / reserving group of every physical cell: (id, live); a ghost record stands for the object its id named
+  {
+    std::vector<int32_t> usingG, resv, hdr;
+    e.readArray(e.dev.p_using, usingG, T.NP); e.readArray(e.dev.p_resv, resv, T.NP);
+    e.readArray(e.dev.g_hdr, hdr, (size_t)(S.maxGroups + hived::GHOST_GROUPS) * hived::GROUP_HDR_WORDS);
+    auto group = [&](int32_t tag, int c, int32_t g) {
+      if (g < 0) return;
+      const int32_t* h = hdr.data() + (size_t)g * hived::GROUP_HDR_WORDS;
+      if (g < S.maxGroups) o.insert(o.end(), {tag, c, g, h[0] != HIVED_GROUP_NONE ? 1 : 0});
+      else o.insert(o.end(), {tag, c, h[hived::GH_ORIGIN] - 1, 0});
+    };
+    for (int c = 0; c < T.NP; c++) group(HIVED_DS_USING_GROUP, c, usingG[c]);
+    for (int c = 0; c < T.NP; c++) group(HIVED_DS_RESERVING_GROUP, c, resv[c]);
+  }
+  {
+    std::vector<int32_t> bad;
+    e.readArray(e.dev.node_bad, bad, S.nNodes);
+    for (int i = 0; i < S.nNodes; i++) if (bad[i]) o.insert(o.end(), {HIVED_DS_BAD_NODE, i});
+  }
+  for (size_t i = 0; i < o.size() && (int64_t)i < cap; i++) out[i] = o[i];
+  return (int64_t)o.size();
 }
 double hived_bench_last_kernel_ms(hived_ctx* ctx) { return ctx->e.lastKernelMs; }
 double hived_bench_total_kernel_ms(hived_ctx* ctx) { return ctx->e.kernelMsTotal; }

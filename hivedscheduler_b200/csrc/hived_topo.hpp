@@ -26,6 +26,7 @@ constexpr int MAXL = 16;            // levels per chain are 1..MAXL-1
 constexpr int MAX_NODE_LEAVES = 64; // leaves below one cluster-view node
 constexpr int MAX_FANOUT = 64;      // children per cell
 constexpr int FL_DUP_SLACK = 16;    // duplicate entries a free-list segment can hold (see fl_cap)
+constexpr int DM_STALE_SLACK = 16;  // stale entries a doomed-bad segment can hold beyond the VC's preassigned cells (dm_cap)
 
 struct TopoError : std::runtime_error {
   int code;
@@ -496,7 +497,11 @@ inline FlatTopo buildTopo(const std::string& text) {
     for (int32_t b : pTops[c]) T.fl_init_data[T.fl_base[c * MAXL + top] + T.fl_init_len[c * MAXL + top]++] = P[b].finalId;
   }
   T.dm_base.assign((size_t)T.nVCs * T.nChains * MAXL, 0); T.dm_cap.assign((size_t)T.nVCs * T.nChains * MAXL, 0);
-  for (size_t k = 0; k < T.dm_base.size(); k++) { T.dm_base[k] = T.dmTotal; T.dm_cap[k] = T.pre_cnt[k]; T.dmTotal += T.pre_cnt[k]; }
+  for (size_t k = 0; k < T.dm_base.size(); k++) {
+    // doomed bad cells bound now (at most one per preassigned cell) plus stale entries (hived_core.h dm_append)
+    const int32_t cap = T.pre_cnt[k] > 0 ? T.pre_cnt[k] + DM_STALE_SLACK : 0;
+    T.dm_base[k] = T.dmTotal; T.dm_cap[k] = cap; T.dmTotal += cap;
+  }
 
   // ------------------------------------------------------------------ cluster views (topology_aware_scheduler.go:158-198)
   auto makeView = [&](std::vector<BCell>& B, const std::vector<std::vector<int32_t>>& lvl, int32_t top, bool cross, int32_t chain, bool isVirtual) -> int32_t {

@@ -27,6 +27,27 @@ double hived_bench_total_kernel_ms(hived_ctx*);
 int64_t hived_bench_kernel_launches(hived_ctx*);
 int hived_bench_num_ctas(hived_ctx*);            /* CTAs the last batch ran on (VC-parallel execution) */
 int hived_bench_set_result_hash(hived_ctx*, int on); /* toggle the running parity hash (HIVED_OPT_NO_RESULT_HASH) */
+
+/* Test hooks: scheduler state that no result or cell snapshot shows but that decides later calls, for comparing two
+ * implementations of hived.h call by call.  Both are host-side reads of the state; neither changes it. */
+uint64_t hived_debug_view_hash(hived_ctx*); /* hash of every cluster view's persisted order */
+/* Fills out[0..min(cap, n)) and returns n, the number of int32 words of the canonical encoding: a sequence of
+ * sections, each starting with its tag, in this order (cells / nodes / VCs / chains are ABI ids, levels 1-based;
+ * empty lists, zero counters and missing map entries are omitted):
+ *   FREE        chain level n cell*n          free cell list, in slice order, duplicates included
+ *   BAD_FREE    chain level n cell*n          bad free cells
+ *   DOOMED_BAD  vc chain level n cell*n       a VC's doomed bad cells
+ *   VC_FREE     vc chain level count          only (vc, chain) pairs the VC has a counter for
+ *   ALL_VC_FREE / TOTAL_LEFT / ALL_VC_DOOMED  chain level count
+ *   USED_PHYSICAL / USED_VIRTUAL  cell n (priority count)*n   used leaf cells per priority, ascending priority
+ *   USING_GROUP / RESERVING_GROUP cell group live  a physical cell's group; live = 0: not the object its name maps to
+ *   BAD_NODE    node */
+enum {
+  HIVED_DS_FREE = 1, HIVED_DS_BAD_FREE = 2, HIVED_DS_DOOMED_BAD = 3, HIVED_DS_VC_FREE = 4, HIVED_DS_ALL_VC_FREE = 5,
+  HIVED_DS_TOTAL_LEFT = 6, HIVED_DS_ALL_VC_DOOMED = 7, HIVED_DS_USED_PHYSICAL = 8, HIVED_DS_USED_VIRTUAL = 9,
+  HIVED_DS_USING_GROUP = 10, HIVED_DS_RESERVING_GROUP = 11, HIVED_DS_BAD_NODE = 12
+};
+int64_t hived_debug_state(hived_ctx*, int32_t* out, int64_t cap);
 #ifdef __cplusplus
 }
 #endif

@@ -11,6 +11,7 @@
 #include <vector>
 
 #include "../include/hived.h"
+#include "../include/hived_bench.h"
 #include "../include/hived_hash.h"
 #include "hived_oracle.hpp"
 
@@ -560,6 +561,81 @@ uint64_t hived_debug_view_hash(hived_ctx* ctx) {
   }
   for (auto& s : ctx->h->opportunisticSchedulers) one(s.second);
   return total;
+}
+
+/* test hook (same encoding as the device library's, include/hived_bench.h): the lists, counters, used-leaf maps, cell
+   groups and bad nodes that decide later calls */
+int64_t hived_debug_state(hived_ctx* ctx, int32_t* out, int64_t cap) {
+  HivedAlgorithm& h = *ctx->h;
+  std::vector<int32_t> o;
+  const int nC = (int)h.chainNames.size(), nV = (int)h.vcNames.size();
+  auto lists = [&](std::initializer_list<int32_t> head, const ChainCellList& ccl) {
+    for (const auto& kv : ccl.m) {
+      if (kv.second.empty()) continue;
+      o.insert(o.end(), head); o.push_back(kv.first); o.push_back((int32_t)kv.second.size());
+      for (const Cell* c : kv.second) o.push_back(c->id);
+    }
+  };
+  auto counters = [&](std::initializer_list<int32_t> head, const std::map<int32_t, int32_t>& m) {
+    for (const auto& kv : m) {
+      if (kv.second == 0) continue;
+      o.insert(o.end(), head); o.push_back(kv.first); o.push_back(kv.second);
+    }
+  };
+  for (int c = 0; c < nC; c++) {
+    auto it = h.freeCellList.find(h.chainNames[c]);
+    if (it != h.freeCellList.end()) lists({HIVED_DS_FREE, c}, it->second);
+  }
+  for (int c = 0; c < nC; c++) {
+    auto it = h.badFreeCells.find(h.chainNames[c]);
+    if (it != h.badFreeCells.end()) lists({HIVED_DS_BAD_FREE, c}, it->second);
+  }
+  for (int v = 0; v < nV; v++) {
+    auto vt = h.vcDoomedBadCells.find(h.vcNames[v]);
+    if (vt == h.vcDoomedBadCells.end()) continue;
+    for (int c = 0; c < nC; c++) {
+      auto it = vt->second.find(h.chainNames[c]);
+      if (it != vt->second.end()) lists({HIVED_DS_DOOMED_BAD, v, c}, it->second);
+    }
+  }
+  for (int v = 0; v < nV; v++) {
+    auto vt = h.vcFreeCellNum.find(h.vcNames[v]);
+    if (vt == h.vcFreeCellNum.end()) continue;
+    for (int c = 0; c < nC; c++) {
+      auto it = vt->second.find(h.chainNames[c]);
+      if (it != vt->second.end()) counters({HIVED_DS_VC_FREE, v, c}, it->second);
+    }
+  }
+  const std::pair<int32_t, const std::map<std::string, std::map<int32_t, int32_t>>*> perChain[] = {
+      {HIVED_DS_ALL_VC_FREE, &h.allVCFreeCellNum}, {HIVED_DS_TOTAL_LEFT, &h.totalLeftCellNum},
+      {HIVED_DS_ALL_VC_DOOMED, &h.allVCDoomedBadCellNum}};
+  for (const auto& t : perChain)
+    for (int c = 0; c < nC; c++) {
+      auto it = t.second->find(h.chainNames[c]);
+      if (it != t.second->end()) counters({t.first, c}, it->second);
+    }
+  auto used = [&](const std::vector<Cell*>& cells, int32_t tag) {
+    for (const Cell* c : cells) {
+      int32_t k = 0;
+      for (const auto& kv : c->used) k += kv.second != 0;
+      if (k == 0) continue;
+      o.insert(o.end(), {tag, c->id, k});
+      for (const auto& kv : c->used) if (kv.second != 0) o.insert(o.end(), {kv.first, kv.second});
+    }
+  };
+  used(h.physicalCells, HIVED_DS_USED_PHYSICAL);
+  used(h.virtualCells, HIVED_DS_USED_VIRTUAL);
+  auto group = [&](int32_t tag, const Cell* c, const Group* g) {
+    if (g == nullptr) return;
+    auto it = h.affinityGroups.find(g->name);
+    o.insert(o.end(), {tag, c->id, g->id, it != h.affinityGroups.end() && it->second == g ? 1 : 0});
+  };
+  for (const Cell* c : h.physicalCells) group(HIVED_DS_USING_GROUP, c, c->usingGroup);
+  for (const Cell* c : h.physicalCells) group(HIVED_DS_RESERVING_GROUP, c, c->reservingOrReservedGroup);
+  for (int i = 0; i < (int)h.nodeNames.size(); i++)
+    if (h.badNodes.count(h.nodeNames[i])) o.insert(o.end(), {HIVED_DS_BAD_NODE, i});
+  for (size_t i = 0; i < o.size() && (int64_t)i < cap; i++) out[i] = o[i];
+  return (int64_t)o.size();
 }
 
 }  // extern "C"

@@ -2,12 +2,17 @@
 """API-level parity fuzz: random Schedule / AddAllocatedPod / DeleteAllocatedPod / DeleteUnallocatedPod calls and node
 health flips on the reference's own test cluster (example/config/design, with its 46 pod specs), through the host
 mirror of internal.SchedulerAlgorithm, on two implementations of include/hived.h in lock step.  After EVERY call the
-results (bind info / victims / wait reason / error class) and every cell's state are compared.  A platform error
+results (bind info / victims / wait reason / error class), every cell's state, the order of every cluster view and the
+hidden state that decides later calls (tests/hidden_state.py: free / bad-free / doomed-bad lists, the cell counters,
+used-leaf maps, the groups of the cells, bad nodes and every group's placement) are compared.  A platform error
 (the reference's panic) ends a run on both sides — the reference leaves its state undefined there.
 
     python tests/fuzz_api.py emu  [first_seed n_seeds n_ops]   device program (1-lane host emulation) vs oracle
     python tests/fuzz_api.py simt [first_seed n_seeds n_ops]   device program (32-lane SIMT emulation) vs oracle
     python tests/fuzz_api.py cuda [first_seed n_seeds n_ops]   libhived_cuda.so vs oracle (GPU box)
+
+Environment: FUZZ_CLUSTER=synthetic (synthetic_fixture instead of the design config), FUZZ_MIX, FUZZ_RENAME and
+FUZZ_FILTERING (the operation mix, see run_seed), FUZZ_JOBS=n (n worker processes; emulations only).
 """
 import copy
 import os
@@ -17,6 +22,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
 sys.path.insert(0, HERE)
+import hidden_state  # noqa: E402
 from conftest import snapshot_bytes  # noqa: E402
 from golden_scenario import load_fixture  # noqa: E402
 from hivedscheduler_b200 import _cabi  # noqa: E402
@@ -66,9 +72,14 @@ def synthetic_fixture():
     return {"design_config": cfg, "pss": pss}
 
 
+def fixture():
+    """The cluster FUZZ_CLUSTER names: "synthetic" (synthetic_fixture), else the reference's design config."""
+    return synthetic_fixture() if os.environ.get("FUZZ_CLUSTER") == "synthetic" else load_fixture()
+
+
 def run_seed(lib_a, lib_b, seed: int, n_ops: int, fx=None, verbose=False):
     """Returns None (no divergence) or a description of the first one."""
-    fx = fx or (synthetic_fixture() if os.environ.get("FUZZ_CLUSTER") == "synthetic" else load_fixture())
+    fx = fx or fixture()
     rng = random.Random(seed)
     cfg = new_config(copy.deepcopy(fx["design_config"]))
     hs = [alg.HivedAlgorithm(cfg, lib=lib, max_groups=1024, max_pods=4096, max_group_leaves=128, max_group_pods=16)
@@ -165,6 +176,10 @@ def run_seed(lib_a, lib_b, seed: int, n_ops: int, fx=None, verbose=False):
             va, vb = (int(h._lib.hived_debug_view_hash(h._ctx)) for h in hs)
             if va != vb:
                 return "seed %d op %d %s: the persisted order of a cluster view differs" % (seed, step, what)
+            # (groups and pods by name: each mirror interns its own ids)
+            d = hidden_state.diff(*(hidden_state.full(h._lib, h._ctx, h._groups.names, h._pods.names) for h in hs))
+            if d:
+                return "seed %d op %d %s: hidden state differs: %s" % (seed, step, what, d)
             if verbose:
                 print(step, what, ra if what.startswith("Schedule") else "")
     finally:
@@ -189,15 +204,32 @@ def main():
         os.makedirs(os.path.dirname(path), exist_ok=True)
         subprocess.check_call(["g++", "-O1", "-g", "-std=c++17", "-fPIC", "-shared", "-o", path, os.path.join(HERE, "emu", src)])
         lib = _cabi.load_library(path)
-    fx = load_fixture()
+    global _JOB
+    _JOB = (lib, oracle, n_ops, fixture())
+    seeds = range(first, first + count)
+    jobs = int(os.environ.get("FUZZ_JOBS", "1"))
     bad = 0
-    for seed in range(first, first + count):
-        d = run_seed(lib, oracle, seed, n_ops, fx)
+    if jobs > 1 and which != "cuda":
+        import multiprocessing
+        with multiprocessing.get_context("fork").Pool(jobs) as pool:  # workers inherit the loaded libraries
+            results = list(pool.imap(_run_job, seeds, chunksize=4))
+    else:
+        results = map(_run_job, seeds)
+    for d in results:
         if d:
             bad += 1
             print("DIVERGED", d, flush=True)
-    print("api fuzz %s vs oracle: %d seeds x %d ops, %d divergences" % (which, count, n_ops, bad))
+    cluster = "synthetic cluster" if os.environ.get("FUZZ_CLUSTER") == "synthetic" else "design config"
+    print("api fuzz %s vs oracle on the %s: %d seeds x %d ops, %d divergences" % (which, cluster, count, n_ops, bad))
     return 1 if bad else 0
+
+
+_JOB = None  # (lib_a, lib_b, n_ops, fixture) of main()
+
+
+def _run_job(seed):
+    lib_a, lib_b, n_ops, fx = _JOB
+    return run_seed(lib_a, lib_b, seed, n_ops, fx)
 
 
 if __name__ == "__main__":

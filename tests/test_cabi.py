@@ -73,3 +73,16 @@ def test_product_fails_loudly_without_a_device():
 def test_missing_extension_is_an_error(tmp_path):
     with pytest.raises(_cabi.MissingExtension):
         _cabi.load_library(str(tmp_path / "libhived_cuda.so"))
+
+
+def test_state_hooks_are_declared_and_exported_by_every_implementation(emu_lib, oracle_lib):
+    """hived_debug_view_hash / hived_debug_state are test hooks of include/hived_bench.h: the product exports them
+    (test_header_symbols_are_bound_and_exported) and so do the implementations the tests compare it with; the section
+    tags of the encoding are the ones tests/hidden_state.py decodes."""
+    import hidden_state
+    assert {"hived_debug_view_hash", "hived_debug_state"} <= set(declared_symbols("hived_bench.h"))
+    for lib in (emu_lib, oracle_lib):
+        assert getattr(lib, "hived_debug_view_hash") is not None and getattr(lib, "hived_debug_state") is not None
+    src = open(os.path.join(ROOT, "include", "hived_bench.h")).read()
+    tags = {m[0]: int(m[1]) for m in re.findall(r"HIVED_DS_([A-Z_]+)\s*=\s*(\d+)", src)}
+    assert tags and tags == {k: getattr(hidden_state, k) for k in tags}
